@@ -198,6 +198,31 @@ def bind_to_gpu_numa_node(local_rank):
   return None
 
 
+DUMP_BUDGET_BYTES = 60 * 10 ** 6   # the arrays of --dump-outputs; with the .npy headers < 64 MB
+DUMP_SEED = 0
+
+
+def dump_outputs(res, out_dir):
+  """Writes the per-env outputs of one step (an engine.StepResult) as DIR/<name>.npy, so that two
+  builds can be compared output for output: reward (float64), step_type, success, status and
+  frames (float32, exact for their integer values), and env_index (float64), the envs they belong
+  to.  When all envs would exceed DUMP_BUDGET_BYTES, the envs are a fixed sample drawn with
+  DUMP_SEED, in ascending order."""
+  import torch
+  os.makedirs(out_dir, exist_ok=True)
+  E = int(res.reward.shape[0])
+  per_env = 8 * 2 + 4 * (3 + res.frames[0].numel())   # reward, env_index; the float32 arrays
+  n = min(E, DUMP_BUDGET_BYTES // per_env)
+  idx = np.arange(E) if n == E else np.sort(np.random.RandomState(DUMP_SEED).choice(E, n, replace=False))
+  rows = torch.as_tensor(idx, device=res.reward.device)
+  arrays = dict(env_index=idx.astype(np.float64))
+  for name in ('reward', 'step_type', 'success', 'status', 'frames'):
+    a = getattr(res, name).index_select(0, rows).cpu().numpy()
+    arrays[name] = a.astype(np.float64 if name == 'reward' else np.float32)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 class Bench(object):
   """One workload on this rank's GPU: engine, frame ring, gather plumbing, timed loops."""
 
@@ -224,6 +249,7 @@ class Bench(object):
     self.n_ring = max(2, int(np.ceil(160e6 / self.frame_bytes)) + 1)
     self.ring = [self.raster.new_frames() for _ in range(self.n_ring)]
     self.gathered, self.peer, self.inflight, self.n_gslots = None, None, [], 2
+    self.last = None   # StepResult of the latest step
     self.gather = args.gather
     if world > 1 and self.gather == 'nccl':
       self._nccl_buffers()
@@ -273,18 +299,18 @@ class Bench(object):
       self.wait_for(lambda it: it[2] == dst)   # everyone is done with the step that last used dst
       if self.gather == 'ce':
         # variant: render into this rank's block, then copy-engine pushes to the peers
-        eng.step(self.actions[t % T], raster, peer.own_slab(dst))
+        self.last = eng.step(self.actions[t % T], raster, peer.own_slab(dst))
         self.inflight.append((peer.push(dst), -1, dst))
       else:
         # the per-env records ride along as ONE all-gather behind the kernel (SURVEY 8e); it is also
         # the completion barrier of the frame stores: it cannot finish before every rank's kernel has
-        eng.step_gather(self.actions[t % T], raster, peer.slot(dst))
+        self.last = eng.step_gather(self.actions[t % T], raster, peer.slot(dst))
         self.inflight.append((dist.all_gather_into_tensor(self.out_all[dst], eng.out_bytes, async_op=True),
                               -1, dst))
       return
     self.wait_for(lambda it: it[1] == slot)    # the gather that last read this ring buffer
     fr = self.ring[slot]
-    eng.step(self.actions[t % T], raster, fr)
+    self.last = eng.step(self.actions[t % T], raster, fr)
     if self.world > 1 and gather:
       # the single collective of the path as a separate NCCL all-gather.  It runs on NCCL's
       # stream and overlaps the next step's compute.
@@ -309,50 +335,41 @@ class Bench(object):
       ms = float(t.item())
     return ms
 
-  def timed_blocks(self, min_seconds, gather=True, t_base=0):
-    """Blocks of exactly `steps` steps, each bracketed by barrier + synchronize and timed with
-    CUDA events (max over ranks), repeated until the timed total reaches `min_seconds`; returns
-    the per-block milliseconds."""
+  def timed_steps(self, gather=True, t_base=0):
+    """Exactly `steps` steps, bracketed by barrier + synchronize and timed with CUDA events (max
+    over ranks); returns the milliseconds."""
     torch = self.torch
-    blocks, total, t = [], 0.0, t_base
-    while True:
-      ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-      self.barrier()
-      ev0.record()
-      for _ in range(self.steps):
-        self.one_step(t, gather)
-        t += 1
-      self.drain()
-      ev1.record()
-      self.barrier()
-      ms = self._max_over_ranks(ev0.elapsed_time(ev1))
-      blocks.append(ms)
-      total += ms
-      if total >= 1e3 * min_seconds or len(blocks) >= 200:
-        return blocks
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    self.barrier()
+    ev0.record()
+    for t in range(t_base, t_base + self.steps):
+      self.one_step(t, gather)
+    self.drain()
+    ev1.record()
+    self.barrier()
+    return self._max_over_ranks(ev0.elapsed_time(ev1))
 
-  def run(self, min_seconds, sampler=None):
-    """Warm-up, the timed blocks, the sharded variant at N > 1 and the render kernel alone."""
+  def run(self, sampler=None, dump_dir=None):
+    """Warm-up, the timed steps, the sharded variant at N > 1 and the render kernel alone.
+    With `dump_dir`, the outputs of the last timed step are written there (dump_outputs)."""
     torch = self.torch
+    if sampler:   # before the warm-up, so that the GPU does not idle right before the timed steps
+      sampler.start()
+      time.sleep(0.3)
     for t in range(self.warmup):
       self.one_step(t)
     self.barrier()
-    if sampler:
-      sampler.start()
-      time.sleep(0.3)
     launches0 = self.eng.launch_count()
-    blocks = self.timed_blocks(min_seconds, True, self.warmup)
-    launches = (self.eng.launch_count() - launches0) // len(blocks)
-    ms = float(np.median(blocks))
+    ms = self.timed_steps(True, self.warmup)
+    launches = self.eng.launch_count() - launches0
     res = dict(value=self.world * self.E * self.steps / (ms * 1e-3), ms_per_step=ms / self.steps,
-               launches=int(launches), timed=dict(
-                   blocks=len(blocks), steps_per_block=self.steps, seconds=sum(blocks) * 1e-3,
-                   ms_per_step_median=ms / self.steps, ms_per_step_min=min(blocks) / self.steps,
-                   ms_per_step_max=max(blocks) / self.steps))
+               launches=int(launches), timed=dict(steps=self.steps, seconds=ms * 1e-3))
+    if dump_dir:
+      # before anything else runs: the render loop below reuses the frame buffers
+      dump_outputs(self.last, dump_dir)
     if self.world > 1:
       # SURVEY 8(e) asks for both numbers: the same steps with the frames left sharded
-      sb = self.timed_blocks(min(min_seconds, 0.5), False, self.T)
-      sms = float(np.median(sb))
+      sms = self.timed_steps(False, self.T)
       res['frames_sharded'] = dict(value=self.world * self.E * self.steps / (sms * 1e-3), unit=UNIT,
                                    ms_per_step=sms / self.steps)
       # the gather's NVLink load: every rank takes in the other ranks' frames each step
@@ -470,8 +487,9 @@ def main():
                   help='comma list of the other BASELINE configs measured in the same run '
                        '(default: c3,c4,c5 at N=1; c4,c5 at N>1; "none" to skip)')
   ap.add_argument('--envs', type=int, default=0, help='override envs per GPU')
-  ap.add_argument('--min-seconds', type=float, default=1.0,
-                  help='the block of --steps timed steps is repeated until this much time is timed')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write the outputs of the last timed step of the headline workload to '
+                       'DIR/<name>.npy (float32 / float64); at N > 1, those of rank 0\'s envs')
   ap.add_argument('--gather', default='peer', choices=['peer', 'ce', 'nccl'],
                   help='N>1 frame gather: stores into peer memory from the render kernel, or a '
                        'separate NCCL all-gather')
@@ -509,7 +527,7 @@ def main():
 
   sampler = ClockSampler(local_rank) if rank == 0 else None
   b = Bench(wl, args, world, rank, local_rank, args.steps, args.warmup, E=args.envs or None)
-  res = b.run(args.min_seconds, sampler)
+  res = b.run(sampler, args.dump_outputs if rank == 0 else None)
   clocks = sampler.stop() if sampler else None
   e2e = None if args.no_e2e else b.e2e()
   collective = ('none' if world == 1 else
@@ -541,7 +559,7 @@ def main():
   if world == 1 and args.also != 'none':
     bi = Bench(wl, args, world, rank, local_rank, min(args.steps, 100), 5, E=args.envs or None,
                max_episode_length=2 ** 31 - 1)
-    r = bi.run(0.3)
+    r = bi.run()
     extra['max_episode_length_inf'] = dict(
         value=r['value'], unit=UNIT, ms_per_step=r['ms_per_step'],
         note='max_episode_length = 2^31-1: envs reset only when the task terminates them')
@@ -555,7 +573,7 @@ def main():
   for key in [k for k in also.split(',') if k and k != 'none' and k != args.workload]:
     w2 = workloads.WORKLOADS[key]()
     b2 = Bench(w2, args, world, rank, local_rank, min(args.steps, 100), 5)
-    r2 = b2.run(min(args.min_seconds, 0.5))
+    r2 = b2.run()
     t2, _ = _traffic(key)
     entry = dict(value=r2['value'], unit=UNIT, ms_per_step=r2['ms_per_step'], n_gpus=world,
                  config=workload_config(w2, b2.E), timed=r2['timed'],

@@ -436,6 +436,33 @@ def sampling_cases(seed=5, n_scenes=12):
   print('sampling.npz: %d config/mode pairs' % (len(blob) // 7))
 
 
+def reference_probes():
+  """reference_probes.npz: the records of tests/reference_probes.py against the reference, keyed
+  '<probe>:<record>', and its public surface under 'surface'."""
+  import importlib
+  import types
+  from spriteworld_b200 import gym_wrapper as own_gym_wrapper
+  # by path: the reference's own `tests` package is ahead of ours on sys.path
+  spec = importlib.util.spec_from_file_location(
+      'reference_probes', os.path.join(ROOT, 'tests', 'reference_probes.py'))
+  probes = importlib.util.module_from_spec(spec)
+  spec.loader.exec_module(probes)
+  if importlib.util.find_spec('gym') is None and importlib.util.find_spec('gymnasium') is None:
+    # the reference's gym_wrapper only builds spaces from specs; gym is absent here
+    gym, spaces = types.ModuleType('gym'), types.ModuleType('gym.spaces')
+    for name in ('Box', 'Discrete', 'Dict', 'Tuple'):
+      setattr(spaces, name, getattr(own_gym_wrapper._MiniSpaces, name))
+    gym.spaces = spaces
+    sys.modules.update({'gym': gym, 'gym.spaces': spaces})
+  sw = lambda name: importlib.import_module('spriteworld.' + name)
+  blob = dict(surface=np.array(json.dumps(probes.public_surface(sw))))
+  for name in sorted(probes.HOST) + sorted(probes.ENGINE):
+    for key, v in probes.run(name, sw).items():
+      blob['%s:%s' % (name, key)] = np.asarray(v)
+  np.savez_compressed(os.path.join(OUT, 'reference_probes.npz'), **blob)
+  print('reference_probes.npz: %d records' % len(blob))
+
+
 def main():
   sampling_cases()
   render_cases()
@@ -451,6 +478,7 @@ def main():
                n_slots=7, action_dtype='int32', frame_envs=(0, 1))
   run_episodes('moving', moving_sprites_config, n_envs=8, n_steps=40, n_slots=4,
                action_dtype='float32', frame_envs=(0,))
+  reference_probes()
 
 
 if __name__ == '__main__':

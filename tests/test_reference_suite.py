@@ -1,129 +1,71 @@
-"""The reference's own test files, run against spriteworld_b200 (CPU tier).
+"""This package against the original Spriteworld package (CPU tier).
 
-`spriteworld` is aliased to `spriteworld_b200`, so every `from spriteworld import ...` in the
-reference's tests/ resolves to this package, unmodified.  The modules that only touch host code
-(factor distributions, sprite generators, shapes, sprites, handcrafted renderers) run as they
-are; the ones that call tasks, action spaces, the PIL renderer or whole environments need the
-device, so here the engine is replaced by the oracle-backed double (tests/oracle_engine.py):
-what is under test is this package's host layer -- task / action compilation, scene packing,
-the plugin protocol, the config modules -- the device arithmetic has its own parity tests
-(`-m gpu`).  Skipped where /root/reference does not exist (the GPU boxes).
+tests/reference_probes.py calls the public API both packages share with seeded inputs;
+tests/golden/reference_probes.npz holds what the original package returned (written by
+tests/golden/make_golden.py).  Here the same probes run against spriteworld_b200 and every record
+must equal the original's.  The probes of modules that drive the engine (tasks, action spaces, the
+PIL renderer, configs, environments, the gym wrapper) run on the oracle-backed double
+(tests/oracle_engine.py): what is under test is this package's host layer -- task / action
+compilation, scene packing, the plugin protocol, the config modules -- the device arithmetic has
+its own parity tests (`-m gpu`).
 """
 import importlib
-import importlib.abc
-import importlib.util
+import json
+import math
 import os
-import sys
-import unittest
 
+import numpy as np
 import pytest
 
-REF_TESTS = os.path.join(os.environ.get('SPRITEWORLD_REFERENCE', '/root/reference'), 'tests')
+from tests import reference_probes as probes
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason='reference tests not present')
-
-
-class _Alias(importlib.abc.MetaPathFinder, importlib.abc.Loader):
-  """spriteworld[.x.y] -> spriteworld_b200[.x.y]"""
-
-  def find_spec(self, name, path, target=None):
-    if name == 'spriteworld' or name.startswith('spriteworld.'):
-      return importlib.util.spec_from_loader(name, self)
-    return None
-
-  def create_module(self, spec):
-    return importlib.import_module('spriteworld_b200' + spec.name[len('spriteworld'):])
-
-  def exec_module(self, module):
-    pass
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_probes.npz')
 
 
-def _third_party_stand_ins():
-  """dm_env (with test_utils) and gym are absent from this image.  The reference's tests get
-  them as views of what the package itself uses in their place: its dm_env surface
-  (spriteworld_b200._dm_env), its minimal gym spaces, and a restatement of dm_env's
-  EnvironmentTestMixin (oracle/refshim/standins/dm_env/test_utils.py)."""
-  import types
-  from oracle.refshim import loader
-  from spriteworld_b200 import _dm_env, gym_wrapper
-  mods = {}
-  if importlib.util.find_spec('dm_env') is None:
-    dm = types.ModuleType('dm_env')
-    for name in ('Environment', 'TimeStep', 'StepType', 'restart', 'transition', 'termination'):
-      setattr(dm, name, getattr(_dm_env, name))
-    specs = types.ModuleType('dm_env.specs')
-    for name in ('Array', 'BoundedArray', 'DiscreteArray'):
-      setattr(specs, name, getattr(_dm_env.specs, name))
-    spec = importlib.util.spec_from_file_location(
-        'dm_env.test_utils', os.path.join(loader._STANDINS, 'dm_env', 'test_utils.py'))
-    test_utils = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(test_utils)
-    dm.specs, dm.test_utils = specs, test_utils
-    mods.update({'dm_env': dm, 'dm_env.specs': specs, 'dm_env.test_utils': test_utils})
-  if importlib.util.find_spec('gym') is None and importlib.util.find_spec('gymnasium') is None:
-    gym = types.ModuleType('gym')
-    spaces = types.ModuleType('gym.spaces')
-    for name in ('Box', 'Discrete', 'Dict', 'Tuple'):
-      setattr(spaces, name, getattr(gym_wrapper._MiniSpaces, name))
-    gym.spaces = spaces
-    mods.update({'gym': gym, 'gym.spaces': spaces})
-  return mods
+def _ours(name):
+  return importlib.import_module('spriteworld_b200.' + name)
 
 
-@pytest.fixture
-def reference_alias():
-  from oracle.refshim import loader
-  loader._patch_aliases()   # np.cast / mock aliases the reference's tests rely on
-  finder = _Alias()
-  sys.meta_path.insert(0, finder)
-  stand_ins = _third_party_stand_ins()
-  sys.modules.update(stand_ins)
-  yield
-  sys.meta_path.remove(finder)
-  for name in stand_ins:
-    sys.modules.pop(name, None)
-  for name in [n for n in sys.modules if n == 'spriteworld' or n.startswith('spriteworld.')]:
-    del sys.modules[name]
+def _same(h, w):
+  """Decoded records: floats to 1e-6 relative (the Clustering reward matches the reference to
+  1e-6, oracle/README.md), everything else exactly."""
+  if isinstance(w, float) or isinstance(h, float):
+    return (type(h) in (int, float) and type(w) in (int, float) and
+            (h == w or math.isclose(h, w, rel_tol=1e-6, abs_tol=1e-12) or (h != h and w != w)))
+  if isinstance(w, list):
+    return isinstance(h, list) and len(h) == len(w) and all(_same(a, b) for a, b in zip(h, w))
+  if isinstance(w, dict):
+    return isinstance(h, dict) and sorted(h) == sorted(w) and all(_same(h[k], w[k]) for k in w)
+  return type(h) is type(w) and h == w
 
 
-def _run(rel):
-  path = os.path.join(REF_TESTS, rel + '.py')
-  spec = importlib.util.spec_from_file_location('reference_' + rel.replace('/', '_'), path)
-  mod = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(mod)
-  suite = unittest.defaultTestLoader.loadTestsFromModule(mod)
-  result = unittest.TestResult()
-  suite.run(result)
-  problems = ['%s: %s' % (t.id(), tb.strip().splitlines()[-1]) for t, tb in
-              result.failures + result.errors]
-  return result.testsRun, problems
+def _compare(name):
+  blob = np.load(GOLDEN, allow_pickle=False)
+  want = {k.split(':', 1)[1]: blob[k] for k in blob.files if k.startswith(name + ':')}
+  have = probes.run(name, _ours)
+  assert want and sorted(have) == sorted(want)
+  bad = []
+  for key, w in sorted(want.items()):
+    h = have[key]
+    if w.dtype.kind == 'U':
+      ok = isinstance(h, str) and _same(json.loads(h), json.loads(str(w)))
+    else:
+      ok = isinstance(h, np.ndarray) and h.dtype == w.dtype and np.array_equal(h, w)
+    if not ok:
+      bad.append('%s: %.300s != %.300s' % (key, h, w))
+  assert not bad, '\n'.join(bad)
 
 
-@pytest.mark.parametrize('rel,n_tests', [
-    ('factor_distributions_test', 39), ('sprite_generators_test', 7), ('shapes_test', 21),
-    ('sprite_test', 16), ('renderers/handcrafted_test', 24)])
-def test_reference_host_tests(reference_alias, rel, n_tests):
-  ran, problems = _run(rel)
-  assert not problems, '\n'.join(problems)
-  assert ran == n_tests
+@pytest.mark.parametrize('name', sorted(probes.HOST))
+def test_host_modules_match_the_reference(name):
+  _compare(name)
 
 
-@pytest.mark.parametrize('rel,n_tests', [
-    ('tasks_test', 85), ('action_spaces_test', 30), ('renderers/pil_renderer_test', 5),
-    ('configs/configs_test', 8), ('environment_test', 7), ('gym_wrapper_test', 2)])
-def test_reference_protocol_tests_on_oracle_engine(reference_alias, monkeypatch, rel, n_tests):
+@pytest.mark.parametrize('name', sorted(probes.ENGINE))
+def test_engine_modules_match_the_reference_on_oracle_engine(monkeypatch, name):
   from tests import oracle_engine
   oracle_engine.install(monkeypatch)
-  ran, problems = _run(rel)
-  assert not problems, '\n'.join(problems)
-  assert ran == n_tests
-
-
-SURFACE_MODULES = [
-    'action_spaces', 'constants', 'environment', 'factor_distributions', 'gym_wrapper', 'shapes',
-    'sprite', 'sprite_generators', 'tasks', 'renderers', 'renderers.abstract_renderer',
-    'renderers.color_maps', 'renderers.handcrafted', 'renderers.pil_renderer',
-    'configs.cobra.common']
+  _compare(name)
 
 
 def test_public_surface_of_the_reference_is_present():
@@ -131,41 +73,19 @@ def test_public_surface_of_the_reference_is_present():
   on and around the path exists under the same name in spriteworld_b200 (demo_ui / run_demo /
   example_run_loop are out of scope, DESIGN.md section 8)."""
   import inspect
-  from oracle.refshim import loader
-  stand_ins = _third_party_stand_ins()
-  sys.modules.update(stand_ins)
-  try:
-    loader.load_reference()
-    missing = []
-    for m in SURFACE_MODULES:
-      ref = importlib.import_module('spriteworld.' + m)
-      ours = importlib.import_module('spriteworld_b200.' + m)
-      for name, obj in vars(ref).items():
-        if name.startswith('_') or inspect.ismodule(obj) or type(obj).__name__ == '_Feature':
-          continue   # private, submodule, `from __future__ import ...`
-        if getattr(obj, '__module__', ref.__name__) != ref.__name__ and (
-            inspect.isclass(obj) or inspect.isfunction(obj)) and m != 'renderers':
-          continue   # imported helper; `renderers` re-exports its classes on purpose
-        if not hasattr(ours, name):
-          missing.append('%s.%s' % (m, name))
-          continue
-        mine = getattr(ours, name)
-        if inspect.isclass(obj):
-          missing += ['%s.%s.%s' % (m, name, a) for a in vars(obj)
-                      if not a.startswith('_') and not hasattr(mine, a)]
-          if '__init__' in vars(obj):
-            want = [p for p in inspect.signature(obj.__init__).parameters if p != 'self']
-            have = [p for p in inspect.signature(mine.__init__).parameters if p != 'self']
-            if want != have[:len(want)]:
-              missing.append('%s.%s(%s)' % (m, name, ', '.join(want)))
-        elif inspect.isfunction(obj):
-          want = list(inspect.signature(obj).parameters)
-          have = list(inspect.signature(mine).parameters)
-          if want != have[:len(want)]:
-            missing.append('%s.%s(%s)' % (m, name, ', '.join(want)))
-    assert not missing, missing
-  finally:
-    for name in stand_ins:
-      sys.modules.pop(name, None)
-    for name in [n for n in sys.modules if n == 'spriteworld' or n.startswith('spriteworld.')]:
-      del sys.modules[name]
+  surface = json.loads(str(np.load(GOLDEN, allow_pickle=False)['surface']))
+  assert surface
+  missing = []
+  for m, name, attrs, params in surface:
+    ours = _ours(m)
+    if not hasattr(ours, name):
+      missing.append('%s.%s' % (m, name))
+      continue
+    mine = getattr(ours, name)
+    missing += ['%s.%s.%s' % (m, name, a) for a in attrs if not hasattr(mine, a)]
+    if params is not None:
+      have = [p for p in inspect.signature(mine.__init__ if inspect.isclass(mine) else mine).parameters
+              if p != 'self']
+      if params != have[:len(params)]:
+        missing.append('%s.%s(%s)' % (m, name, ', '.join(params)))
+  assert not missing, missing
